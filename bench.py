@@ -43,7 +43,36 @@ def parse_args():
     ap.add_argument("--ref-frames", type=int, default=2, help="frames per step of the CPU reference arm")
     ap.add_argument("--cpu-sample", type=int, default=48, help="frames of the cpu_baseline sample (b200 arm)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the packed keypoint payloads of the last timed step (device-resident and end-to-end) "
+                         "to DIR/<name>.npy, float32")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the b200 path")
+    return args
+
+
+def payload_as_received(packed, keep):
+    """Packed payload rows [..., keep*row + keep + 1] with the person slots beyond each image's count zeroed: the parser
+    leaves them unwritten and LitePosePipeline.unpack() never reads them."""
+    import numpy as np
+    a = np.array(packed, dtype=np.float32)
+    row = (a.shape[-1] - 1 - keep) // keep
+    for r in a.reshape(-1, a.shape[-1]):
+        p = min(int(r[-1]), keep)
+        r[p * row:keep * row] = 0
+        r[keep * row + p:keep * row + keep] = 0
+    return a
+
+
+def dump_outputs(directory, arrays):
+    """One float32 .npy per array: the same arguments give the same inputs, so two builds compare output for output."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 def workload_config(args, n_gpus):
@@ -648,11 +677,13 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        _, parsed = step(x_dev, plant)
+        packed, parsed = step(x_dev, plant)
     if parsed is not None:
         torch.cuda.current_stream().wait_event(parsed)
     e1.record()
     barrier()
+    # the payload buffers are reused by the steps below: keep the last timed step's result now
+    last_packed = packed.cpu().numpy() if args.dump_outputs else None
     t_dev = max_over_ranks(e0.elapsed_time(e1) * 1e-3)
     clocks = sampler.stop() if rank == 0 else None
     value = world * B * args.steps / t_dev
@@ -695,6 +726,11 @@ def main():
     t_e2e = max(t_e2e, t_wall)
     e2e_value = world * B * args.steps / t_e2e
     host_out = last_host[0]
+    if args.dump_outputs and rank == 0:
+        # packed: [N, keep*J*(3+T) + keep + 1] of rank 0 (keypoints, scores, person count; LitePosePipeline.unpack);
+        # e2e_packed: [ranks, N, ...] as collect() hands it to rank 0's host
+        dump_outputs(args.dump_outputs, {"packed": payload_as_received(last_packed, pipe.keep),
+                                         "e2e_packed": payload_as_received(host_out.numpy(), pipe.keep)})
 
     if rank != 0:
         if world > 1:

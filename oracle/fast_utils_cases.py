@@ -47,3 +47,13 @@ GOLDEN_CASES = [
     (10, dict(people=0, clutter=3), 0.1, 5, 30, 1.0),
     (11, dict(people=2, h=16, w=16, n=3), 0.1, 1, 30, 1.0),      # window 1: every pixel >= threshold is a peak
 ]
+
+
+def random_case(seed):
+    """The randomised sweep (threshold 0.1, window 5, max_count 30, tag threshold 1.0, JOINT_ORDER_17) for seeds
+    RANDOM_SEEDS; images may exceed the reference's 10-entry arrays, the checks skip those."""
+    return make_case(seed, people=1 + seed % 6, spread=[2.0, 0.7, 0.3][seed % 3], tagnoise=[0.05, 0.3][seed % 2],
+                     plateau=seed % 5 == 0, clutter=[0, 5, 12][seed % 3])
+
+
+RANDOM_SEEDS = range(100, 160)

@@ -43,6 +43,45 @@ def sd_digest(sd):
     return h.hexdigest()
 
 
+def tensor_digest(t):
+    """sha256 over a tensor's or array's dtype, shape and bytes: equal digests <=> equal arrays (for finite values)."""
+    a = t.detach().cpu().contiguous().numpy() if torch.is_tensor(t) else np.ascontiguousarray(t)
+    h = hashlib.sha256()
+    h.update(("%s%s" % (a.dtype.str, a.shape)).encode())
+    h.update(a.tobytes())
+    return h.hexdigest()
+
+
+# the second target of the sub-network transfer check (besides LitePose-S): three stages deep, one block in the last
+SUBNET_TINY_ARCH = {
+    "img_size": 256, "input_channel": 16, "deconv_setting": [16, 24, 24],
+    "backbone_setting": [{"num_blocks": 2, "stride": 2, "channel": 16, "block_setting": [[6, 7]] * 2},
+                         {"num_blocks": 3, "stride": 2, "channel": 24, "block_setting": [[6, 7]] * 3},
+                         {"num_blocks": 2, "stride": 2, "channel": 40, "block_setting": [[6, 7]] * 2},
+                         {"num_blocks": 1, "stride": 1, "channel": 64, "block_setting": [[6, 7]] * 1}]}
+
+
+def golden_subnet_transfer():
+    """The reference's own transfer() (weight_transfer.py, function bodies executed where the file lies) from a
+    LitePose-L (seed 3) into LitePose-S and SUBNET_TINY_ARCH (seed 4): one digest per tensor of the target's state
+    dict (the full tensors are tens of MB)."""
+    import ast
+    path = os.path.join(refshim.REF_ROOT, "weight_transfer.py")
+    fns = [n for n in ast.parse(open(path).read()).body if isinstance(n, ast.FunctionDef) and n.name.startswith("transfer")]
+    cfg = get_cfg()
+    ns = {"cfg": cfg}
+    exec(compile(ast.Module(body=fns, type_ignores=[]), "weight_transfer_fns", "exec"), ns)
+    big = refshim.build_reference_model(cfg, get_arch("L"), seed=3)
+    blob = {}
+    for name, arch in (("S", get_arch("S")), ("tiny", SUBNET_TINY_ARCH)):
+        small = refshim.build_reference_model(cfg, arch, seed=4)
+        ns["transfer"](big, small, arch)
+        want = small.state_dict()
+        blob[name + "_keys"] = np.array(list(want))
+        blob[name + "_digest"] = np.array([tensor_digest(v) for v in want.values()])
+    np.savez_compressed(os.path.join(OUT, "subnet_transfer.npz"), **blob)
+
+
 def golden_model():
     ns = refshim.load()
     # (1) tiny arch: weights + per-layer activations committed
@@ -313,6 +352,8 @@ if __name__ == "__main__":
         golden_parser_shared_tag()
         golden_glue_multiscale()
         golden_glue_cfgs()
+    elif len(sys.argv) > 1 and sys.argv[1] == "--subnet-transfer":
+        golden_subnet_transfer()
     else:
         golden_model()
         golden_glue()
@@ -321,5 +362,6 @@ if __name__ == "__main__":
         golden_glue_multiscale()
         golden_glue_cfgs()
         golden_munkres()
+        golden_subnet_transfer()
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)))

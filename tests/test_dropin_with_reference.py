@@ -1,6 +1,8 @@
-"""CPU, build container only (skipped where /root/reference is absent): the sys.path shadowing
-of INTEGRATION.md §1 resolves `models.pose_mobilenet` / `core.group` / `utils.transforms` to this repo and
-`core.inference`, `utils.zipreader` ... to the unmodified reference, and the reference glue runs on our module's outputs."""
+"""CPU: the sys.path shadowing of INTEGRATION.md §1 resolves `models.pose_mobilenet` / `core.group` /
+`utils.transforms` to this repo and `core.inference`, `utils.zipreader` ... to the reference, and the reference glue
+runs on our module's outputs.  The reference is a stand-in tree with the reference's package layout (written per test):
+`lib/models` a regular package that imports its members, `lib/core` and `lib/utils` namespace packages, `_init_paths.py`
+putting `lib` at the front of sys.path; its `core.inference` is the glue restatement oracle/glue_ref.py."""
 import os
 import subprocess
 import sys
@@ -8,7 +10,32 @@ import sys
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+
+STAND_IN = {
+    "_init_paths.py": "import os.path, sys\n"
+                      "lib = os.path.join(os.path.dirname(__file__), 'lib')\n"
+                      "if lib not in sys.path:\n    sys.path.insert(0, lib)\n",
+    "lib/models/__init__.py": "import models.pose_higher_hrnet\nimport models.pose_mobilenet\n",
+    "lib/models/pose_higher_hrnet.py": "def get_pose_net(cfg, is_train, **kwargs):\n    raise NotImplementedError\n",
+    "lib/models/pose_mobilenet.py": "raise ImportError('the stand-in reference model must never be imported')\n",
+    "lib/core/group.py": "raise ImportError('the stand-in reference parser must never be imported')\n",
+    "lib/core/inference.py": "from dataset.transforms import FLIP_CONFIG\n"
+                             "from oracle.glue_ref import aggregate_results\n"
+                             "from oracle.glue_ref import multi_stage_outputs as get_multi_stage_outputs\n",
+    "lib/utils/transforms.py": "def fliplr_joints(joints, joints_vis, width, matched_parts):\n"
+                               "    raise NotImplementedError\n",
+    "lib/utils/zipreader.py": "def imread(filename):\n    raise NotImplementedError\n",
+}
+
+
+@pytest.fixture
+def ref_tree(tmp_path):
+    base = tmp_path / "reference"
+    for rel, text in STAND_IN.items():
+        path = base / rel
+        path.parent.mkdir(parents=True, exist_ok=True)
+        path.write_text(text)
+    return str(base)
 
 SCRIPT = r'''
 import sys, types
@@ -42,9 +69,8 @@ print("dropin ok")
 '''
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "lib", "core")), reason="reference tree not present")
-def test_sys_path_shadowing():
-    r = subprocess.run([sys.executable, "-c", SCRIPT % {"ref": REF, "root": ROOT}], capture_output=True, text=True,
+def test_sys_path_shadowing(ref_tree):
+    r = subprocess.run([sys.executable, "-c", SCRIPT % {"ref": ref_tree, "root": ROOT}], capture_output=True, text=True,
                        timeout=300)
     assert r.returncode == 0 and "dropin ok" in r.stdout, r.stdout + r.stderr
 
@@ -73,26 +99,25 @@ print("init_paths dropin ok")
 '''
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "lib", "core")), reason="reference tree not present")
 @pytest.mark.parametrize("how", ["sitecustomize", "runner"])
-def test_dropin_survives_init_paths(tmp_path, how):
+def test_dropin_survives_init_paths(tmp_path, ref_tree, how):
     """ADVICE r1: valid.py's `import _init_paths` inserts <reference>/lib at sys.path[0] AFTER PYTHONPATH /
     sitecustomize, and <reference>/lib/models is a regular package - plain path shadowing loses and the model would
     silently be the stock eager one.  The meta-path drop-in (litepose_b200/dropin.py) must win in both launch modes."""
     script = tmp_path / "check_like_valid.py"
-    script.write_text(CHECK % {"ref": REF, "root": ROOT})
+    script.write_text(CHECK % {"ref": ref_tree, "root": ROOT})
     env = dict(os.environ)
     if how == "sitecustomize":
         env["PYTHONPATH"] = os.pathsep.join([os.path.join(ROOT, "litepose_b200", "dropin_site"), ROOT])
         # cwd = reference root so that `import _init_paths` resolves like for `python valid.py`
-        cmd = [sys.executable, "-c", "import sys; sys.path.insert(0, %r); exec(open(%r).read())" % (REF, str(script))]
+        cmd = [sys.executable, "-c", "import sys; sys.path.insert(0, %r); exec(open(%r).read())" % (ref_tree, str(script))]
     else:
         env["PYTHONPATH"] = ROOT
         # the runner puts the script's directory first (as `python script.py` does); _init_paths lives beside valid.py
         link = tmp_path / "ref"
-        os.symlink(REF, link)
+        os.symlink(ref_tree, link)
         runner_script = tmp_path / "run_in_ref.py"
-        runner_script.write_text("import sys; sys.path.insert(0, %r)\n" % REF + CHECK % {"ref": REF, "root": ROOT})
+        runner_script.write_text("import sys; sys.path.insert(0, %r)\n" % ref_tree + CHECK % {"ref": ref_tree, "root": ROOT})
         cmd = [sys.executable, "-m", "litepose_b200.dropin", str(runner_script)]
-    r = subprocess.run(cmd, capture_output=True, text=True, timeout=300, env=env, cwd=REF)
+    r = subprocess.run(cmd, capture_output=True, text=True, timeout=300, env=env, cwd=ref_tree)
     assert r.returncode == 0 and "init_paths dropin ok" in r.stdout, r.stdout + r.stderr

@@ -321,20 +321,19 @@ TRAIN: {LR: 4e-3, WD: 1e-4}
     assert cfg2.DATASET.NUM_JOINTS == 15 and cfg2.MODEL.NUM_JOINTS == 15 and cfg2.TEST.SCALE_FACTOR == [0.5, 1, 2]
     with pytest.raises(KeyError):
         load_experiment(str(path), opts=["TEST.NO_SUCH_KEY", "1"])
-    ref_yaml = "/root/reference/experiments/crowd_pose/mobilenet/mobile.yaml"
-    if os.path.exists(ref_yaml):               # the reference's own file (build container only)
-        cfg3, _ = load_experiment(ref_yaml, superconfig="S")
-        for sec in ("MODEL", "LOSS", "DATASET", "TEST"):
-            for k, v in ref[sec].items():
-                if k in skip:
-                    continue
-                got = cfg3[sec][k]
-                if isinstance(v, (list, tuple)):
-                    assert list(got) == list(v), (sec, k)
-                elif isinstance(v, dict):        # the file may carry more keys (PRETRAINED_LAYERS ...)
-                    assert all(list(got[k2]) == list(v2) if isinstance(v2, list) else got[k2] == v2 for k2, v2 in v.items()), (sec, k)
-                else:
-                    assert got == v, (sec, k)
+    # the reference's own experiment file (experiments/crowd_pose/mobilenet/mobile.yaml, stored verbatim)
+    cfg3, _ = load_experiment(os.path.join(ROOT, "tests", "golden", "crowd_pose_mobile.yaml"), superconfig="S")
+    for sec in ("MODEL", "LOSS", "DATASET", "TEST"):
+        for k, v in ref[sec].items():
+            if k in skip:
+                continue
+            got = cfg3[sec][k]
+            if isinstance(v, (list, tuple)):
+                assert list(got) == list(v), (sec, k)
+            elif isinstance(v, dict):        # the file may carry more keys (PRETRAINED_LAYERS ...)
+                assert all(list(got[k2]) == list(v2) if isinstance(v2, list) else got[k2] == v2 for k2, v2 in v.items()), (sec, k)
+            else:
+                assert got == v, (sec, k)
 
 
 def test_valid_synthetic_cli_dry_run(tmp_path):

@@ -1,7 +1,7 @@
 """SURVEY 8(f) row 4: sub-network extraction from a larger checkpoint (reference weight_transfer.py:75-146)."""
-import ast
 import os
 
+import numpy as np
 import pytest
 import torch
 
@@ -9,7 +9,7 @@ from litepose_b200.config import get_arch, get_cfg
 from litepose_b200.lib.models.pose_mobilenet import get_pose_net
 from litepose_b200.subnet import extract_subnet, extract_subnet_state_dict
 
-REF = "/root/reference/weight_transfer.py"
+GOLD = os.path.join(os.path.dirname(__file__), "golden", "subnet_transfer.npz")
 
 
 def _big(seed=0):
@@ -38,27 +38,23 @@ def test_prefix_slices_and_strict_load(arch):
         extract_subnet_state_dict(sd, sup)
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference checkout not present")
 def test_matches_reference_transfer():
-    """the reference's own transfer() (function bodies executed from weight_transfer.py where it lies) on reference modules"""
-    from oracle import refshim
-    src = open(REF).read()
-    fns = [n for n in ast.parse(src).body if isinstance(n, ast.FunctionDef) and n.name.startswith("transfer")]
+    """against the reference's own transfer() (weight_transfer.py) from the same LitePose-L into LitePose-S and a tiny
+    arch: tests/golden/subnet_transfer.npz holds a digest of every tensor it produced (oracle/make_golden.py)"""
+    from litepose_b200.synth import randomize_bn_
+    from oracle.make_golden import SUBNET_TINY_ARCH, tensor_digest
+    g = np.load(GOLD)
     cfg = get_cfg()
-    ns = {"cfg": cfg}
-    exec(compile(ast.Module(body=fns, type_ignores=[]), "weight_transfer_fns", "exec"), ns)
-    big = refshim.build_reference_model(cfg, get_arch("L"), seed=3)
-    tiny = {"img_size": 256, "input_channel": 16, "deconv_setting": [16, 24, 24],
-            "backbone_setting": [{"num_blocks": 2, "stride": 2, "channel": 16, "block_setting": [[6, 7]] * 2},
-                                 {"num_blocks": 3, "stride": 2, "channel": 24, "block_setting": [[6, 7]] * 3},
-                                 {"num_blocks": 2, "stride": 2, "channel": 40, "block_setting": [[6, 7]] * 2},
-                                 {"num_blocks": 1, "stride": 1, "channel": 64, "block_setting": [[6, 7]] * 1}]}
-    for arch in (get_arch("S"), tiny):
-        small = refshim.build_reference_model(cfg, arch, seed=4)
-        ns["transfer"](big, small, arch)
-        want = small.state_dict()
-        got = extract_subnet_state_dict(big.state_dict(), want)
-        for k in want:
+    torch.manual_seed(3)                               # the reference model's initialisation (oracle/refshim.py)
+    big = randomize_bn_(get_pose_net(cfg, False, get_arch("L")), 1).eval().state_dict()
+    for name, arch in (("S", get_arch("S")), ("tiny", SUBNET_TINY_ARCH)):
+        keys = [str(k) for k in g[name + "_keys"]]
+        want = dict(zip(keys, (str(d) for d in g[name + "_digest"])))
+        torch.manual_seed(4)
+        target = randomize_bn_(get_pose_net(cfg, False, arch), 1).eval().state_dict()
+        assert list(target) == keys
+        got = extract_subnet_state_dict(big, target)
+        for k in keys:
             if k.endswith("num_batches_tracked"):
                 continue                                   # the reference leaves the target's own counter
-            assert torch.equal(got[k], want[k]), k
+            assert tensor_digest(got[k]) == want[k], (name, k)
